@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the batched inflate / gzip / PNG decode path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python bench.py --strong cfg4|cfg5 --gpus N        (one batch over N GPUs through dbg_decode_batch_packed_multi)
 
 One "step" = one pass of the hot path over one batch of synthetic input. The headline workload is BASELINE.json
@@ -220,12 +220,8 @@ def run_reference(args):
 # ------------------------------------------------------------------------ PNG ---
 def _gen_png(spec):
     """spec = (index, w, h, forced filter or None). stb_write when the tooling is there, else the own encoder."""
-    i, w, h, filt = spec
     from debigulator_b200 import corpus
-    if corpus.stb_available():
-        return corpus.png_stb(i, w, h, filt)
-    img = corpus.gradient_noise_rgba(w, h, 0x706E6700 + i)
-    return corpus.write_png(img, filt=(i % 6 - 1) if filt is None else filt, single_block=True), img.tobytes()
+    return corpus.png_bench(*spec)
 
 
 def png_corpus(w, h, n_unique, filt, share_tag=None, rank=0, world=1, barrier=None):
@@ -253,7 +249,7 @@ def png_corpus(w, h, n_unique, filt, share_tag=None, rank=0, world=1, barrier=No
     return uniq
 
 
-def bench_png(ctx, dbg, dev, torch, name, n, w, h, uniq, peak, steps=3, e2e=True, cpu=True, world=1, max_over_ranks=lambda x: x,
+def bench_png(ctx, dbg, dev, torch, name, n, w, h, uniq, peak, steps, e2e=True, cpu=True, world=1, max_over_ranks=lambda x: x,
               barrier=lambda: None, e2e_images=None):
     from debigulator_b200 import corpus
     n_unique = len(uniq)
@@ -346,19 +342,18 @@ def bench_png(ctx, dbg, dev, torch, name, n, w, h, uniq, peak, steps=3, e2e=True
         a4 = (in_off[:ne], in_size[:ne], out_off[:ne], out_cap[:ne])
         ctx.decode_packed(dbg.api.KIND_PNG, h_in, a4[0], a4[1], h_out, a4[2], a4[3])
         barrier()
-        reps = 2
         t0 = time.perf_counter()
-        for _ in range(reps):
+        for _ in range(steps):
             osz, st = ctx.decode_packed(dbg.api.KIND_PNG, h_in, a4[0], a4[1], h_out, a4[2], a4[3])
         torch.cuda.synchronize()
-        dt1 = max_over_ranks(time.perf_counter() - t0) / reps
+        dt1 = max_over_ranks(time.perf_counter() - t0) / steps
         assert int(st.sum()) == 0 and int(osz.sum()) == ne * rgba, f"{name}: e2e failures"
         for k in (0, 1, ne // 2, ne - 1):
             assert h_out[k * rgba:(k + 1) * rgba].tobytes() == uniq[k % n_unique][1], f"{name}: e2e pixel mismatch"
         # two calls in flight (dbg_pipe_*): the batch as two sub-batches, one's ramp under the other's downloads
         ctx.trim()
         h_out[:] = 0
-        dt, osz, st, pipe_launches = e2e_pipelined(dbg, dev.index, dbg.api.KIND_PNG, h_in, a4[0], a4[1], h_out, a4[2], a4[3], reps,
+        dt, osz, st, pipe_launches = e2e_pipelined(dbg, dev.index, dbg.api.KIND_PNG, h_in, a4[0], a4[1], h_out, a4[2], a4[3], steps,
                                                    barrier, max_over_ranks)
         assert int(st.sum()) == 0 and int(osz.sum()) == ne * rgba, f"{name}: pipelined e2e failures"
         for k in (0, 1, ne // 2 - 1, ne // 2, ne - 1):
@@ -375,7 +370,7 @@ def bench_png(ctx, dbg, dev, torch, name, n, w, h, uniq, peak, steps=3, e2e=True
         ct = max_over_ranks(time.perf_counter() - t0)
         out["e2e"] = {"value": world * ne * w * h / dt / 1e6, "unit": "Mpix/s", "rgba_GBps": world * ne * rgba / dt / 1e9,
                       "ms_per_step": dt * 1e3, "images_per_gpu": ne, "h2d_bytes_per_step": int(e_in), "d2h_bytes_per_step": int(ne * rgba),
-                      "steps": reps, "calls_in_flight": 2,
+                      "steps": steps, "calls_in_flight": 2,
                       "api": "dbg_pipe_submit / dbg_pipe_wait (kind=PNG): every step's batch as two packed sub-batches of the same "
                              "pinned host arenas, two in flight",
                       "single_call": {"value": world * ne * w * h / dt1 / 1e6, "unit": "Mpix/s", "ms_per_step": dt1 * 1e3,
@@ -430,6 +425,26 @@ def e2e_pipelined(dbg, dev_index, kind, h_in_np, in_off, in_size, h_out_np, out_
     launches = (pipe.kernel_launches() - l0) / steps
     pipe.close()
     return dt, osz, st, launches
+
+
+DUMP_SAMPLE = 1 << 22  # decoded bytes kept by --dump-outputs: 16 MiB as float32
+DUMP_SEED = 20240601
+
+
+def dump_outputs(out_dir, torch, d_out, d_out_size, d_status, n, size, stride):
+    """What a caller of the device-resident gzip path receives from one call, as float arrays: every member's status
+    and output size, and the decoded bytes at a fixed, seeded sample of positions of the n x `size` payloads (the whole
+    output is n x 1 MiB). The positions are written too, so that two dumps can be compared position by position."""
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(DUMP_SEED)
+    pos = np.sort(rng.choice(n * size, size=min(DUMP_SAMPLE, n * size), replace=False)).astype(np.int64)
+    flat = torch.from_numpy((pos // size) * stride + pos % size).to(d_out.device)
+    arrays = {"status": d_status.cpu().numpy().astype(np.float64),
+              "out_size": d_out_size.cpu().numpy().astype(np.float64),
+              "payload_sample": d_out[flat].cpu().numpy().astype(np.float32),
+              "payload_sample_pos": pos.astype(np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ----------------------------------------------------------------------- ours ---
@@ -530,7 +545,8 @@ def run_ours(args):
     for _ in range(args.warmup):
         step_device()
     barrier()
-    verify()
+    if args.warmup:
+        verify()
     d_out.zero_()
     launches0 = ctx.kernel_launches
     ctx.profile_enable(True)
@@ -550,27 +566,28 @@ def run_ours(args):
     ctx.profile_enable(False)
     launches = ctx.kernel_launches - launches0
     verify()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, torch, d_out, d_out_size, d_status, n, size, stride)
     value = world * n * size * args.steps / (dev_ms / 1e3) / 1e9
 
     # ---- end to end through the packed host API (pinned host arenas)
     hin_np, hout_np = h_in.numpy(), h_out.numpy()
-    e2e_steps = max(1, min(args.steps, 5))
     ctx.decode_packed(dbg.api.KIND_GZ, hin_np, in_off, in_size, hout_np, out_off, out_cap)
     barrier()
     t0 = time.perf_counter()
-    for _ in range(e2e_steps):
+    for _ in range(args.steps):
         osz, st = ctx.decode_packed(dbg.api.KIND_GZ, hin_np, in_off, in_size, hout_np, out_off, out_cap)
     torch.cuda.synchronize()
     e2e_s = max_over_ranks(time.perf_counter() - t0)
     assert int(st.sum()) == 0 and int(osz.sum()) == out_total
     for k in (0, 1, 2, 3, n - 1):
         assert hout_np[k * stride:k * stride + size].tobytes() == uniq[k % N_UNIQUE][1], "e2e payload mismatch"
-    e2e_single = world * out_total * e2e_steps / e2e_s / 1e9
+    e2e_single = world * out_total * args.steps / e2e_s / 1e9
     # the same with two calls in flight (dbg_pipe_*: the batch as two sub-batches, one's ramp under the other's downloads)
     ctx.trim()
     hout_np[:] = 0
     pdt, osz, st, pipe_launches = e2e_pipelined(dbg, local, dbg.api.KIND_GZ, hin_np, in_off, in_size, hout_np, out_off, out_cap,
-                                                max(2, e2e_steps), barrier, max_over_ranks)
+                                                args.steps, barrier, max_over_ranks)
     assert int(st.sum()) == 0 and int(osz.sum()) == out_total
     for k in (0, 1, 2, 3, n // 2 - 1, n // 2, n - 1):
         assert hout_np[k * stride:k * stride + size].tobytes() == uniq[k % N_UNIQUE][1], "pipelined e2e payload mismatch"
@@ -613,7 +630,7 @@ def run_ours(args):
                 box = [e2e_n]
             dist.broadcast_object_list(box, src=0)
             e2e_n = box[0]
-        png = bench_png(ctx, dbg, dev, torch, "cfg3", args.png_images, PNG_W, PNG_H, uniq3, peak, e2e=True,
+        png = bench_png(ctx, dbg, dev, torch, "cfg3", args.png_images, PNG_W, PNG_H, uniq3, peak, args.steps, e2e=True,
                         cpu=(rank == 0 and world == 1 and not args.no_cpu), world=world, max_over_ranks=max_over_ranks, barrier=barrier,
                         e2e_images=e2e_n)
         del uniq3
@@ -621,19 +638,19 @@ def run_ours(args):
         uniq4 = png_corpus(PNG4_W, PNG4_H, min(PNG4_UNIQUE, args.png_large), 4, "cfg4" if world > 1 else None, rank, world, barrier)
         ctx.trim()
         torch.cuda.empty_cache()
-        png_large = bench_png(ctx, dbg, dev, torch, "cfg4 (forced Paeth)", args.png_large, PNG4_W, PNG4_H, uniq4, peak, e2e=(world == 1),
+        png_large = bench_png(ctx, dbg, dev, torch, "cfg4 (forced Paeth)", args.png_large, PNG4_W, PNG4_H, uniq4, peak, args.steps, e2e=(world == 1),
                               cpu=(rank == 0 and world == 1 and not args.no_cpu), world=world, max_over_ranks=max_over_ranks, barrier=barrier)
         del uniq4
         ctx.trim()
         torch.cuda.empty_cache()
     bmp = cfg5 = cfg1 = None
     if args.bmp and rank == 0 and world == 1:
-        bmp = bench_bmp(ctx, dev, torch, args.bmp)
-        bmp["sprite_sheet"] = bench_sprites(ctx, dev, torch)
+        bmp = bench_bmp(ctx, dev, torch, args.bmp, args.steps)
+        bmp["sprite_sheet"] = bench_sprites(ctx, dev, torch, args.steps)
     if args.cfg5 and rank == 0 and world == 1:
-        cfg5 = bench_cfg5(ctx, dev, torch, args.cfg5)
+        cfg5 = bench_cfg5(ctx, dev, torch, args.cfg5, args.steps)
     if args.cfg1 and rank == 0 and world == 1:
-        cfg1 = bench_cfg1(ctx, no_cpu=args.no_cpu)
+        cfg1 = bench_cfg1(ctx, args.steps, no_cpu=args.no_cpu)
 
     # ---- CPU baseline: the reference C on this box's host cores (rank 0, N=1 only)
     cpu = None
@@ -680,10 +697,10 @@ def run_ours(args):
                        "l2": "inputs+outputs per step (%.1f GB) exceed the 126 MB L2; no explicit flush" % ((comp_bytes + out_total) / 1e9),
                        "parallelism": f"{world} independent shard(s), no collective"},
             "e2e": {"value": e2e_val, "unit": UNIT, "h2d_bytes_per_step": int(in_total + 64), "d2h_bytes_per_step": int(out_span),
-                    "steps": max(2, e2e_steps), "ms_per_step": pdt * 1e3, "calls_in_flight": 2,
+                    "steps": args.steps, "ms_per_step": pdt * 1e3, "calls_in_flight": 2,
                     "api": "dbg_pipe_submit / dbg_pipe_wait (kind=gzip): every step's batch as two packed sub-batches of the same "
                            "pinned host arenas, two in flight",
-                    "single_call": {"value": e2e_single, "unit": UNIT, "ms_per_step": e2e_s / e2e_steps * 1e3, "steps": e2e_steps,
+                    "single_call": {"value": e2e_single, "unit": UNIT, "ms_per_step": e2e_s / args.steps * 1e3, "steps": args.steps,
                                     "api": "dbg_decode_batch_packed(kind=gzip), one blocking call per step"},
                     "kernel_launches_per_step": pipe_launches,
                     "link_ceiling": pcie},
@@ -714,7 +731,7 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
-def bench_cfg1(ctx, no_cpu=False):
+def bench_cfg1(ctx, steps, no_cpu=False):
     """BASELINE config 1: the two bundled files as batches of one through the scalar-sized path (wall clock,
     host buffers in, host buffers out), next to the reference C on one core."""
     gold = os.path.join(ROOT, "tests", "golden")
@@ -726,7 +743,7 @@ def bench_cfg1(ctx, no_cpu=False):
             r = fn()
         assert r[0][0] == 1
         ts = []
-        for _ in range(10):
+        for _ in range(steps):
             t0 = time.perf_counter()
             fn()
             ts.append(time.perf_counter() - t0)
@@ -748,7 +765,7 @@ def _gen_cfg5(i):
     return g, len(d), zlib.crc32(d)
 
 
-def bench_cfg5(ctx, dev, torch, n, n_unique=64):
+def bench_cfg5(ctx, dev, torch, n, steps, n_unique=64):
     """BASELINE config 5 shape, scaled to one GPU: gzip members of 64 KiB-16 MiB (log-uniform), eight
     compressibility classes, device-resident. The long members take the block-split path (DESIGN.md 4.3)."""
     uniq = pool_map(_gen_cfg5, list(range(n_unique)))
@@ -790,7 +807,6 @@ def bench_cfg5(ctx, dev, torch, n, n_unique=64):
             assert zlib.crc32(data) == uniq[k][2], f"cfg5 payload mismatch in member {k}"
             checked += 1
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    steps = 3
     e0.record()
     for _ in range(steps):
         step()
@@ -808,7 +824,7 @@ def bench_cfg5(ctx, dev, torch, n, n_unique=64):
             "block_split_streams_per_step": (after[0] - before[0]) // (steps + 2), "block_split_fallbacks": after[1] - before[1]}
 
 
-def bench_bmp(ctx, dev, torch, n, w=2048, h=2048):
+def bench_bmp(ctx, dev, torch, n, steps, w=2048, h=2048):
     """decode_BMP / encode_BMP on n bottom-up w x h files (SURVEY.md 8(f) rank 4): the one kernel of the
     library that is plain HBM traffic (every pixel read once, written once)."""
     from debigulator_b200 import corpus
@@ -847,7 +863,6 @@ def bench_bmp(ctx, dev, torch, n, w=2048, h=2048):
             fn()
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        steps = 10
         e0.record()
         for _ in range(steps):
             fn()
@@ -876,7 +891,7 @@ def bench_bmp(ctx, dev, torch, n, w=2048, h=2048):
                          "algorithmic_bytes_per_launch": alg, "encode_achieved": alg / (res["encode"] / 1e3) / 1e9}}
 
 
-def bench_sprites(ctx, dev, torch, n=1000, w=512, h=512):
+def bench_sprites(ctx, dev, torch, steps, n=1000, w=512, h=512):
     """Sprite-sheet tiling (SURVEY.md 8(f) rank 4, intent of concat_pngs.c:81-100): n decoded w x h RGBA8 images into one
     sheet of ceil(sqrt(n)) columns; plain HBM traffic (every image pixel read once, every sheet pixel written once)."""
     rgba = w * h * 4
@@ -892,11 +907,11 @@ def bench_sprites(ctx, dev, torch, n=1000, w=512, h=512):
         r, c = ctx.tile_sprites_device(d_img, off, n, w, h, 0, True, d_sheet, stream=stream)
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for _ in range(5):
+    for _ in range(steps):
         ctx.tile_sprites_device(d_img, off, n, w, h, 0, True, d_sheet, stream=stream)
     e1.record()
     torch.cuda.synchronize()
-    ms = e0.elapsed_time(e1) / 5
+    ms = e0.elapsed_time(e1) / steps
     sheet = d_sheet.view(rows * h, cols * w * 4)
     for i in (0, 1, cols, n - 1):  # spot check: tile i against its image
         rr, cc = divmod(i, cols)
@@ -975,7 +990,8 @@ def run_strong(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5,
+                    help="timed steps of every GPU measurement (device-resident, end-to-end, secondary lines)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--members", type=int, default=N_MEMBERS)
@@ -988,7 +1004,13 @@ def main():
     ap.add_argument("--bmp", type=int, default=64, help="number of 2048x2048 BMP files in the BMP line (0 = skip)")
     ap.add_argument("--strong", default=None, choices=["cfg4", "cfg5"], help="one batch over --gpus devices (dbg_multi_*)")
     ap.add_argument("--images", type=int, default=0, help="--strong: items in the batch")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step of the headline workload returned to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.strong):
+        ap.error("--dump-outputs writes the outputs of the headline GPU workload: not with --impl reference or --strong")
     if args.impl == "reference":
         run_reference(args)
     elif args.strong:

@@ -54,13 +54,23 @@ def build_library(force=False, verbose=False):
 
 
 STBGEN = os.path.join(HERE, "tools", "libstbgen.so")
+CORPUS_TOOLS = os.path.join(HERE, "tools", "libcorpus_tools.so")
 REF_SRC = "/root/reference/src"
 
 
+def build_corpus_tools():
+    """The corpus's own single-block fixed-Huffman encoder (tools/fixed_deflate.c). Returns the library path."""
+    src = os.path.join(HERE, "tools", "fixed_deflate.c")
+    if not os.path.exists(CORPUS_TOOLS) or os.path.getmtime(src) > os.path.getmtime(CORPUS_TOOLS):
+        subprocess.check_call(["gcc", "-O2", "-fPIC", "-shared", src, "-o", CORPUS_TOOLS])
+    return CORPUS_TOOLS
+
+
 def build_tools():
-    """Corpus tooling (not product code): the synthetic-PNG writer, compiled against the reference's vendored
-    stb_write.h where it lies. Returns the library path, or None when neither the reference tree nor a prebuilt
-    library is there (the GPU box uses the prebuilt one)."""
+    """Corpus tooling (not product code): the corpus's own encoder, and the synthetic-PNG writer compiled against the
+    reference's vendored stb_write.h where it lies. Returns the stb library path, or None when neither the reference
+    tree nor a prebuilt library is there."""
+    build_corpus_tools()
     src = os.path.join(HERE, "tools", "stb_gen.c")
     if os.path.isdir(REF_SRC):
         if not os.path.exists(STBGEN) or os.path.getmtime(src) > os.path.getmtime(STBGEN):

@@ -7,9 +7,7 @@ stb_image_write produces: one IDAT, filter forced or adaptive), so the decoder
 under test never sees its own encoder.
 """
 import ctypes
-import os
 import struct
-import subprocess
 import zlib
 
 import numpy as np
@@ -21,12 +19,8 @@ def _tools():
     """Builds (gcc, once) and loads the corpus tools: the single-block fixed-Huffman encoder."""
     global _TOOLS
     if _TOOLS is None:
-        here = os.path.dirname(os.path.abspath(__file__))
-        src = os.path.join(here, "tools", "fixed_deflate.c")
-        so = os.path.join(here, "tools", "libcorpus_tools.so")
-        if not os.path.exists(so) or os.path.getmtime(src) > os.path.getmtime(so):
-            subprocess.check_call(["gcc", "-O2", "-fPIC", "-shared", src, "-o", so])
-        L = ctypes.CDLL(so)
+        from .build import build_corpus_tools
+        L = ctypes.CDLL(build_corpus_tools())
         L.dbg_fixed_deflate.argtypes = [ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p, ctypes.c_size_t]
         L.dbg_fixed_deflate.restype = ctypes.c_size_t
         _TOOLS = L
@@ -285,11 +279,17 @@ def write_png(img, filt=-1, level=6, strategy=zlib.Z_FIXED, idat_split=0, color_
     return out + _chunk(b"IEND", b"")
 
 
-def png_cfg3(i, w=1024, h=1024):
-    """BASELINE config 3 image i: forced filter i%6-1 (-1 = adaptive). Returns (png bytes, rgba bytes).
-    Written by this module's own encoder (tools/fixed_deflate.c): the stream shape stb writes, not stb itself."""
+def png_cfg3(i, w=1024, h=1024, filt=None):
+    """BASELINE config 3 image i: filter forced to i%6-1 (-1 = adaptive) unless `filt` says otherwise. Returns (png bytes,
+    rgba bytes). Written by this module's own encoder (tools/fixed_deflate.c): the stream shape stb writes, not stb itself."""
     img = gradient_noise_rgba(w, h, 0x706E6700 + i)
-    return write_png(img, filt=i % 6 - 1, single_block=True), img.tobytes()
+    return write_png(img, filt=(i % 6 - 1) if filt is None else filt, single_block=True), img.tobytes()
+
+
+def png_bench(i, w=1024, h=1024, filt=None):
+    """BASELINE config 3 / 4 image i as the benchmark times it: written by stb_image_write when that tooling is built
+    (png_stb), else by this module's own encoder of the same stream shape (png_cfg3). Same pixels either way."""
+    return (png_stb if stb_available() else png_cfg3)(i, w, h, filt)
 
 
 def png_stb(i, w=1024, h=1024, filt=None):

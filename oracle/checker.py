@@ -1,6 +1,7 @@
 """The checker tests, smoke() and bench.py's CPU legs use: the unmodified
 reference (oracle/_ref/libref.so, kind "reference") when it is available, else
-the plain-C restatement (oracle/liboracle.so, kind "port").
+the plain-C restatement (oracle/liboracle.so, kind "port"), which
+tests/test_oracle.py pins to the reference's own outputs in tests/golden.
 
 TEST INFRASTRUCTURE ONLY (see oracle/__init__.py).
 """
@@ -42,6 +43,27 @@ def decode_bmp(data: bytes, out_size: int = None):
 
 def encode_bmp(rgba: bytes, w: int, h: int):
     return _impl().encode_bmp(rgba, w, h)
+
+
+def stb_png(pixels: bytes, w: int, h: int, comp: int = 4, filt: int = -1) -> bytes:
+    """A PNG of the shape stb_write.h writes (one IDAT, zlib header 78 5E, one final fixed-Huffman block): the
+    reference's own stb_write.h when it is available, else the corpus's encoder (debigulator_b200/tools/fixed_deflate.c)."""
+    if reflib.available():
+        return reflib.stb_png(pixels, w, h, comp, filt)
+    import numpy as np
+    from debigulator_b200 import corpus
+    img = np.frombuffer(bytes(pixels), np.uint8).reshape(h, w, comp)
+    return corpus.write_png(img, filt=filt, single_block=True)
+
+
+def stb_zlib(data: bytes, quality: int = 8) -> bytes:
+    """A zlib stream of the shape stb_write.h writes (78 5E, one final fixed-Huffman block, Adler-32); see stb_png."""
+    if reflib.available():
+        return reflib.stb_zlib(data, quality)
+    import struct
+    import zlib
+    from debigulator_b200 import corpus
+    return b"\x78\x5e" + corpus.fixed_block_deflate(data) + struct.pack(">I", zlib.adler32(bytes(data)) & 0xFFFFFFFF)
 
 
 class TimedRunner:
