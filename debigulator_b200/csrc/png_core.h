@@ -28,6 +28,8 @@
 
 #ifdef DBG_SIMT_EMU
 static inline uint32_t atomicAdd(uint32_t *p, uint32_t v) { uint32_t o = *p; *p = o + v; return o; }
+static inline uint32_t atomicXor(uint32_t *p, uint32_t v) { uint32_t o = *p; *p = o ^ v; return o; }
+struct uint4 { uint32_t x, y, z, w; };
 #endif
 
 namespace dbg {
@@ -213,6 +215,32 @@ DBG_DEV bool scan_enqueue(ScanQueues *q, const uint8_t *p, uint64_t n, uint8_t *
     }
     return true;
 }
+
+// One segment task (png_tasks_kernel, uniform call): its contribution to the CRC of its chunk, XOR-ed into the chunk's
+// accumulator, and its copy.
+DBG_DEV void scan_task_run(const CrcTables *T, uint32_t lane_k, const ScanTask &k, BigChunk *big)
+{
+    const uint32_t ln = (uint32_t)simt::lane();
+    if (k.big != SCAN_NONE) {
+        uint32_t st = crc_state_warp(T, lane_k, k.src, k.len, k.first ? 0xffffffffu : 0u);
+        st = gf2_mulmod(gf2_xpow_bytes(k.bytes_after), st);
+        if (ln == 0) atomicXor(&big[k.big].acc, st);
+    }
+    if (k.dst) {
+        if ((((uintptr_t)k.src | (uintptr_t)k.dst) & 15) == 0) {
+            const uint4 *s4 = (const uint4 *)k.src;
+            uint4 *d4 = (uint4 *)k.dst;
+            for (uint32_t i = ln; i < k.len / 16; i += 32) d4[i] = s4[i];
+            for (uint32_t i = (k.len & ~15u) + ln; i < k.len; i += 32) k.dst[i] = k.src[i];
+        } else {
+            for (uint32_t i = ln; i < k.len; i += 32) k.dst[i] = k.src[i];
+        }
+    }
+}
+
+// png_verify_kernel: the recombined CRC of a large chunk against the stored one (decode_png.c:1341-1348), once every
+// segment task has run. A chunk the walk never got to the end of is not armed and fails on its own account.
+DBG_DEV bool big_chunk_crc_bad(const BigChunk &c) { return c.armed && (c.acc ^ 0xffffffffu) != c.expected; }
 
 // --------------------------------------------------------------- chunk walk ----
 DBG_DEV uint32_t be32(const uint8_t *p)

@@ -87,10 +87,11 @@ static inline PngLayout png_layout(uint8_t *base, uint64_t n, uint64_t total_in,
     return l;
 }
 
-// Pass A (one CTA): per-image buffer sizes from IHDR (the same fixed-offset read
-// as decode_png_get_width_height, decode_png.c:662-671) and their exclusive
-// prefix sums. An image whose IHDR disagrees with the caller's rgba size gets
-// no scan buffer; png_scan_warp fails it with the reference's own check.
+// Pass A (one CTA): per-image buffer sizes and their exclusive prefix sums. The
+// scanline buffer is sized for any IHDR whose w*h*4 is the caller's rgba size:
+// the walk accepts every such IHDR and the last one sets the inflate capacity
+// (decode_png.c:965-968), so png_scan_kernel sets s_cap once the walk is done;
+// w >= 1 bounds h by rgba/4.
 constexpr int PLAN_THREADS = 1024;
 __global__ void __launch_bounds__(PLAN_THREADS) png_plan_kernel(PngBatch b)
 {
@@ -109,16 +110,11 @@ __global__ void __launch_bounds__(PLAN_THREADS) png_plan_kernel(PngBatch b)
         uint32_t i = base + t;
         uint64_t zc = 0, sc = 0, est = 0;
         if (i < b.n) {
-            uint64_t size = b.in_size[i];
-            zc = png_align(size + 16, 16);
-            if (size >= 33) {
-                const uint8_t *f = b.in_base + b.in_off[i];
-                uint64_t w = be32(f + 16), h = be32(f + 20);
-                uint64_t rgba = w * h * 4;
-                if (rgba == b.rgba_size[i] && rgba + h + 1 < (1ull << 32) && w >= 1 && h >= 1) {
-                    est = rgba + h + 1;  // decode_png.c:965-968
-                    sc = png_align(est + 16, 16);
-                }
+            zc = png_align(b.in_size[i] + 16, 16);
+            const uint64_t rgba = b.rgba_size[i];
+            if (rgba >= 4 && rgba < (1ull << 32)) {
+                est = rgba + rgba / 4 + 1;
+                sc = png_align(est + 16, 16);
             }
         }
         sh_z[t] = zc;
@@ -138,7 +134,7 @@ __global__ void __launch_bounds__(PLAN_THREADS) png_plan_kernel(PngBatch b)
             const bool z_fits = carry_z + sh_z[t] <= b.lay.idat_bytes, s_fits = carry_s + sh_s[t] <= b.lay.scan_bytes;
             b.lay.z_off[i] = z_fits ? (uint64_t)(uintptr_t)(b.lay.idat + (carry_z + sh_z[t] - zc)) : 0ull;  // absolute address
             b.lay.s_off[i] = s_fits ? carry_s + sh_s[t] - sc : 0ull;
-            b.lay.s_cap[i] = s_fits ? est : 0ull;  // inflate's recipient_size, decode_png.c:803-804
+            b.lay.s_cap[i] = s_fits ? est : 0ull;  // room; png_scan_kernel narrows it to inflate's recipient_size
             b.lay.z_size[i] = 0;
             b.lay.s_size[i] = 0;
             b.lay.inf_status[i] = 0;
@@ -179,6 +175,8 @@ __global__ void __launch_bounds__(SCAN_WARPS * 32) png_scan_kernel(PngBatch b)
             b.lay.z_size[i] = zs;
             b.lay.pre_status[i] = st;
             b.lay.info[i] = info;
+            // recipient_size from the last IHDR the walk accepted (decode_png.c:803-804, 965-968)
+            if (st == ST_OK && b.lay.s_cap[i]) b.lay.s_cap[i] = (uint64_t)info.w * info.h * 4 + info.h + 1;
         }
         simt::syncwarp();
     }
@@ -201,21 +199,7 @@ __global__ void __launch_bounds__(SCAN_WARPS * 32) png_tasks_kernel(PngBatch b)
         if (t >= total) break;
         const ScanTask k = b.lay.queues.tasks[t];
         if (k.len == 0) continue;
-        if (k.big != SCAN_NONE) {
-            uint32_t st = crc_state_warp(&tables, lane_k, k.src, k.len, k.first ? 0xffffffffu : 0u);
-            st = gf2_mulmod(gf2_xpow_bytes(k.bytes_after), st);
-            if (ln == 0) atomicXor(&b.lay.queues.big[k.big].acc, st);
-        }
-        if (k.dst) {
-            if ((((uintptr_t)k.src | (uintptr_t)k.dst) & 15) == 0) {
-                const uint4 *s4 = (const uint4 *)k.src;
-                uint4 *d4 = (uint4 *)k.dst;
-                for (uint32_t i = ln; i < k.len / 16; i += 32) d4[i] = s4[i];
-                for (uint32_t i = (k.len & ~15u) + ln; i < k.len; i += 32) k.dst[i] = k.src[i];
-            } else {
-                for (uint32_t i = ln; i < k.len; i += 32) k.dst[i] = k.src[i];
-            }
-        }
+        scan_task_run(&tables, lane_k, k, b.lay.queues.big);
         simt::syncwarp();
     }
 }
@@ -228,7 +212,7 @@ __global__ void png_verify_kernel(PngBatch b)
     if (nbig > b.lay.queues.big_cap) nbig = b.lay.queues.big_cap;
     if (i >= nbig) return;
     const BigChunk c = b.lay.queues.big[i];
-    if (c.armed && (c.acc ^ 0xffffffffu) != c.expected) atomicMax(&b.lay.pre_status[c.img], (uint32_t)ST_PNG_CRC);
+    if (big_chunk_crc_bad(c)) atomicMax(&b.lay.pre_status[c.img], (uint32_t)ST_PNG_CRC);
 }
 
 // Pass C2 (one CTA): un-filter work items. An image that decoded so far gets one item per 32-row

@@ -455,7 +455,28 @@ struct PngArgs {
     uint32_t status[32];
     uint32_t crc_only;   // when set: just CRC `size` bytes of `file`
     uint32_t crc[32];
+    dbg::ScanQueues *q;  // non-null: the walk defers large chunks (phase 0), the tasks run one by one (phase 1), then
+    uint32_t phase;      // inflate + un-filter (phase 2), as png_scan_kernel / png_tasks_kernel / the later passes do
+    dbg::ScanTask task;
+    dbg::PngInfo info;
+    uint64_t zs;
+    const uint8_t *zp;
 };
+static void png_decode_rest(PngArgs *a, uint32_t &st)
+{
+    const dbg::PngInfo info = a->info;
+    uint64_t est = (uint64_t)info.w * info.h * 4 + info.h + 1, ssize = 0;
+    st = dbg::inflate_warp(a->ism, a->zp, a->zs, a->scan, est, &ssize);
+    simt::syncwarp();  // a kernel boundary in the product: the last deferred match store of one lane is read by another below
+    if (st == dbg::ST_OK) {
+        uint64_t need = (uint64_t)info.h * ((uint64_t)info.w * info.bpp + 1);
+        if (a->scan[0] > 4) st = dbg::ST_PNG_FILTER;
+        else if (ssize < need) st = dbg::ST_PNG_SHORT;
+        else if (info.bpp == 4) dbg::png_unfilter_warp<4>(a->usm, a->scan, info.w, info.h, a->out, nullptr, 0);
+        else if (info.bpp == 3) dbg::png_unfilter_warp<3>(a->usm, a->scan, info.w, info.h, a->out, nullptr, 0);
+        else dbg::png_unfilter_warp<1>(a->usm, a->scan, info.w, info.h, a->out, a->file + info.plte_off, info.plte_size);
+    }
+}
 static void png_body(void *p)
 {
     PngArgs *a = (PngArgs *)p;
@@ -467,36 +488,39 @@ static void png_body(void *p)
         a->crc[l] = dbg::crc32_warp(a->tables, lane_k, a->file, a->size);
         return;
     }
-    dbg::PngInfo info;
-    info.w = info.h = info.bpp = 0;
-    uint64_t zs = 0;
-    const uint8_t *zp = a->zbuf;
-    uint32_t st = dbg::png_scan_warp(a->tables, lane_k, a->file, a->size, a->rgba_size, a->zbuf, a->zcap, &info, &zs, &zp,
-                                     nullptr, 0);
-    if (st == dbg::ST_OK) {
-        uint64_t est = (uint64_t)info.w * info.h * 4 + info.h + 1, ssize = 0;
-        st = dbg::inflate_warp(a->ism, zp, zs, a->scan, est, &ssize);
-        simt::syncwarp();  // a kernel boundary in the product: the last deferred match store of one lane is read by another below
-        if (st == dbg::ST_OK) {
-            uint64_t need = (uint64_t)info.h * ((uint64_t)info.w * info.bpp + 1);
-            if (a->scan[0] > 4) st = dbg::ST_PNG_FILTER;
-            else if (ssize < need) st = dbg::ST_PNG_SHORT;
-            else if (info.bpp == 4) dbg::png_unfilter_warp<4>(a->usm, a->scan, info.w, info.h, a->out, nullptr, 0);
-            else if (info.bpp == 3) dbg::png_unfilter_warp<3>(a->usm, a->scan, info.w, info.h, a->out, nullptr, 0);
-            else dbg::png_unfilter_warp<1>(a->usm, a->scan, info.w, info.h, a->out, a->file + info.plte_off, info.plte_size);
-        }
+    uint32_t st = dbg::ST_OK;
+    if (a->phase == 1) {
+        dbg::scan_task_run(a->tables, lane_k, a->task, a->q->big);
+        return;
     }
+    if (a->phase == 0) {
+        dbg::PngInfo info;
+        info.w = info.h = info.bpp = 0;
+        uint64_t zs = 0;
+        const uint8_t *zp = a->zbuf;
+        st = dbg::png_scan_warp(a->tables, lane_k, a->file, a->size, a->rgba_size, a->zbuf, a->zcap, &info, &zs, &zp, a->q, 0);
+        simt::syncwarp();
+        if (l == 0) {
+            a->info = info;
+            a->zs = zs;
+            a->zp = zp;
+        }
+        simt::syncwarp();
+    }
+    if (st == dbg::ST_OK && (a->phase == 2 || !a->q)) png_decode_rest(a, st);
     a->status[l] = st;
 }
 
-extern "C" uint32_t emu_png_decode(const uint8_t *file, uint64_t size, uint8_t *out, uint64_t rgba_size, int reverse)
+static uint32_t png_decode_impl(const uint8_t *file, uint64_t size, uint8_t *out, uint64_t rgba_size, int misalign, int reverse,
+                                dbg::ScanQueues *q)
 {
     PngArgs a;
     memset(&a, 0, sizeof(a));
-    uint8_t *fcopy = (uint8_t *)aligned_alloc(16, (size + 64 + 15) & ~(uint64_t)15);
-    memset(fcopy, 0xA5, (size + 64 + 15) & ~(uint64_t)15);
-    memcpy(fcopy, file, size);
-    a.file = fcopy;
+    const uint64_t arena = (size + 64 + 16 + 15) & ~(uint64_t)15;
+    uint8_t *fcopy = (uint8_t *)aligned_alloc(16, arena);
+    memset(fcopy, 0xA5, arena);
+    memcpy(fcopy + (misalign & 15), file, size);
+    a.file = fcopy + (misalign & 15);
     a.size = size;
     a.out = out;
     a.rgba_size = rgba_size;
@@ -509,11 +533,54 @@ extern "C" uint32_t emu_png_decode(const uint8_t *file, uint64_t size, uint8_t *
     uint64_t scan_cap = (rgba_size + rgba_size / 4 + 64 + 15) & ~(uint64_t)15;
     a.scan = (uint8_t *)aligned_alloc(16, scan_cap);
     memset(a.scan, 0x77, scan_cap);
+    a.q = q;
     simt::run_warp(png_body, &a, reverse);
     uint32_t st = a.status[0];
     for (int i = 1; i < 32; i++)
         if (a.status[i] != st) st = 0x1000 | i;
+    if (q && st < 0x1000) {
+        // png_tasks_kernel, then png_verify_kernel: the verdict of the walk is raised to 13 by a bad large chunk
+        const uint32_t total = *q->ntasks < q->task_cap ? *q->ntasks : q->task_cap;
+        a.phase = 1;
+        for (uint32_t t = 0; t < total; t++) {
+            a.task = q->tasks[reverse ? total - 1 - t : t];
+            if (a.task.len) simt::run_warp(png_body, &a, reverse);
+        }
+        const uint32_t nbig = *q->nbig < q->big_cap ? *q->nbig : q->big_cap;
+        for (uint32_t i = 0; i < nbig; i++)
+            if (dbg::big_chunk_crc_bad(q->big[i]) && st < dbg::ST_PNG_CRC) st = dbg::ST_PNG_CRC;
+        if (st == dbg::ST_OK) {
+            a.phase = 2;
+            simt::run_warp(png_body, &a, reverse);
+            st = a.status[0];
+            for (int i = 1; i < 32; i++)
+                if (a.status[i] != st) st = 0x1000 | i;
+        }
+    }
     free(fcopy); free(a.tables); free(a.ism); free(a.usm); free(a.zbuf); free(a.scan);
+    return st;
+}
+
+extern "C" uint32_t emu_png_decode(const uint8_t *file, uint64_t size, uint8_t *out, uint64_t rgba_size, int reverse)
+{
+    return png_decode_impl(file, size, out, rgba_size, 0, reverse, nullptr);
+}
+
+// The same with the walk's segment queues (png_task_cap / png_big_cap of a batch of this one file unless the caps are
+// given), the file at `misalign` bytes past a 16-byte boundary. The tasks run in queue order, or in reverse order with
+// the lanes. *ntasks / *nbig: what the walk enqueued.
+extern "C" uint32_t emu_png_decode_queued(const uint8_t *file, uint64_t size, uint8_t *out, uint64_t rgba_size, int misalign,
+                                          int reverse, uint32_t task_cap, uint32_t big_cap, uint32_t *ntasks, uint32_t *nbig)
+{
+    if (!task_cap) task_cap = (uint32_t)(4 * (size / dbg::SCAN_SEG) + 64);
+    if (!big_cap) big_cap = (uint32_t)(size / dbg::SCAN_SEG + 16);
+    std::vector<dbg::ScanTask> tasks(task_cap);
+    std::vector<dbg::BigChunk> big(big_cap);
+    uint32_t counters[2] = {0, 0};
+    dbg::ScanQueues q{tasks.data(), &counters[0], task_cap, big.data(), &counters[1], big_cap};
+    const uint32_t st = png_decode_impl(file, size, out, rgba_size, misalign, reverse, &q);
+    *ntasks = counters[0];
+    *nbig = counters[1];
     return st;
 }
 
